@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- IMU windows/sec of the batched closed-form preintegration hot path (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload v1_10k_200|v2_100k_400]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload v1_10k_200|v2_100k_400] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic IMU windows (cpi_b200/synth.py, seed 20260924).
 Default workload = BASELINE.json configs[1]: 10 000 windows x 200 samples, CPI model 1 (mean + Jacobians + covariance),
@@ -20,6 +20,9 @@ reference's own CPU implementation timed on this box's host cores, rank 0, N = 1
 host entry point with pinned HOST buffers: H2D + kernel + D2H inside the timed region), clocks, gpu_launches.
 `--impl reference` times the reference's CPU path (oracle/_ref when it was compiled, else the oracle port) on all host
 threads on a bounded sample of the same workload.
+`--dump-outputs DIR` writes what the timed CUDA path returned in its last timed step as DIR/<name>.npy (records for the
+preintegration workloads, e / H1 / H2 for the factor ones).  The inputs are seeded, so two builds run with the same arguments
+can be compared output for output.
 """
 import argparse
 import json
@@ -70,6 +73,20 @@ NCU_TRAFFIC = {   # dram__bytes_read.sum + dram__bytes_write.sum per launch of t
 # (model 2 executes ~55 % of the survey's 15 kflop/sample contract -- RK4 applied directly to the consumed Discrete_J_b columns -- so its
 # contract fraction overstates the pipe utilisation; DESIGN.md section 4)
 NCU_FP64_PIPE_PCT = {"v1_10k_200": 43.8, "v2_100k_400": 49.7, "v1_125k_200": 50.6, "v1_1m_200_fp32": 21.6}
+DUMP_BUDGET = 60 << 20     # bytes of --dump-outputs payload per run (stays under 64 MB with the .npy headers)
+
+
+def dump_outputs(dirname, arrays):
+    """Write each array as dirname/<name>.npy.  Above DUMP_BUDGET in all, every array keeps the same fixed, seeded sample of rows
+    (the arrays of one call share their row count), so that dumps of two builds stay comparable row for row."""
+    arrays = {k: v.cpu().numpy() if hasattr(v, "cpu") else np.asarray(v) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_BUDGET:
+            keep = max(1, int(len(a) * DUMP_BUDGET / total))
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -162,18 +179,18 @@ def run_reference(args, wl):
     from cpi_b200 import synth
     cores = synth.usable_cpus()
     if wl.get("single"):
-        # SURVEY 8(d) config 1: one window, reference CpiV1 on ONE thread, median of >= 1000 repeats
+        # SURVEY 8(d) config 1: one window, reference CpiV1 on ONE thread, median over the timed steps
         from oracle.oracle import Oracle, Reference
         impl, kind = (Reference(), "reference") if Reference.available() else (Oracle(), "port")
         S, L = synth.make_windows(1, wl["ns"], rate=wl["rate"], special=False)
         ts = []
-        for _ in range(1200):
+        for _ in range(args.warmup + args.steps):
             t0 = time.perf_counter(); impl.preintegrate(wl["model"], S, L, synth.SIGMAS, 0, ns=wl["ns"], nthreads=1); ts.append(time.perf_counter() - t0)
-        ms = 1e3 * float(np.median(ts[200:]))
-        print(json.dumps({"impl": "reference", "metric": "imu_windows_per_sec", "value": 1e3 / ms, "unit": "windows/s", "n_gpus": args.gpus, "steps": 1000, "warmup": 200,
+        ms = 1e3 * float(np.median(ts[args.warmup:]))
+        print(json.dumps({"impl": "reference", "metric": "imu_windows_per_sec", "value": 1e3 / ms, "unit": "windows/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
                           "ms_per_step": ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
                           "config": config_dict(wl, args.gpus),
-                          "cpu_baseline": {"value": 1e3 / ms, "unit": "windows/s", "cores": 1, "kind": kind, "sample": "1 window x 100 samples, median of 1000 repeats (includes ~3 us of ctypes call overhead)"},
+                          "cpu_baseline": {"value": 1e3 / ms, "unit": "windows/s", "cores": 1, "kind": kind, "sample": f"1 window x 100 samples, median of {args.steps} repeats (includes ~3 us of ctypes call overhead)"},
                           "e2e": {"value": 1e3 / ms, "unit": "windows/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}), flush=True)
         return
     # bounded sample: calibrate on a small run, then size each step for ~5 s of CPU work (all usable host threads)
@@ -197,7 +214,7 @@ def run_reference(args, wl):
     print(json.dumps(line), flush=True)
 
 
-def run_factor(args, wl, emit=True, cpu=True):
+def run_factor(args, wl, emit=True, cpu=True, dump=None):
     """configs[4]: K3 (ImuFactorCPIv1::evaluateError batched) over a 5k-keyframe chain.  HBM-write bound: 4 496 algorithmic
     bytes per factor (776 in, 3 720 out); at 5k factors the launch is ~10 us, i.e. launch-latency sized."""
     from cpi_b200 import synth
@@ -249,6 +266,8 @@ def run_factor(args, wl, emit=True, cpu=True):
     torch.cuda.synchronize()
     launches = capi.launch_count() - launches0
     ms = float(np.mean([a.elapsed_time(b) for a, b in evs]))
+    if dump:
+        dump_outputs(dump, dict(zip(("e", "H1", "H2"), outs)))
     peaks, how = measured_peaks()
     ach = 4496.0 * n / (ms * 1e-3) * 1e-9
     hX, hR, hL = (torch.from_numpy(a).pin_memory() for a in (X, rec, L))
@@ -356,7 +375,7 @@ def _pin_to_gpu_numa_node(self, torch):
 Ctx.pin_to_gpu_numa_node = _pin_to_gpu_numa_node
 
 
-def measure_preint(ctx, name, args, steps, warmup, distinct=None, e2e=True, cpu=False, clocks=True):
+def measure_preint(ctx, name, args, steps, warmup, distinct=None, e2e=True, cpu=False, clocks=True, dump=None):
     """One workload of the preintegration path on this process' GPU (all ranks call it together).  `distinct`: generate only
     that many distinct windows on the host and tile them on the device (host generation is ~0.5 ms per window; the kernel does not
     care, and the resident set still exceeds L2) -- the headline workload always uses all-distinct windows."""
@@ -458,6 +477,8 @@ def measure_preint(ctx, name, args, steps, warmup, distinct=None, e2e=True, cpu=
         total_ms = float(t.item())
     ms_per_step = total_ms / steps
     value = world * n / (ms_per_step * 1e-3)
+    if dump and rank == 0:
+        dump_outputs(dump, {"records": gathers[(warmup + steps - 1) % NG].reshape(-1, rd)})      # every rank's records at N > 1
 
     peaks, how = measured_peaks()
     flops = wl["flops_per_sample"] * ns * n          # algorithmic flops per launch (SURVEY 8d contract)
@@ -564,7 +585,7 @@ def measure_preint(ctx, name, args, steps, warmup, distinct=None, e2e=True, cpu=
     return out
 
 
-def measure_single(ctx, args, wl):
+def measure_single(ctx, args, wl, steps=50, dump=None):
     """configs[0]: ONE 100-sample window -- for the GPU arm this is launch latency (one CTA, three lanes)."""
     import torch
     from cpi_b200 import preint, synth
@@ -575,11 +596,13 @@ def measure_single(ctx, args, wl):
     for _ in range(20):
         preint.preintegrate(1, dS, dL, synth.SIGMAS, 0, ns=wl["ns"], out=out, stream=stream)
     torch.cuda.synchronize()
-    evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(50)]
+    evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
     for a, b in evs:
         a.record(stream); preint.preintegrate(1, dS, dL, synth.SIGMAS, 0, ns=wl["ns"], out=out, stream=stream); b.record(stream)
     torch.cuda.synchronize()
     ms = float(np.median([a.elapsed_time(b) for a, b in evs]))
+    if dump:
+        dump_outputs(dump, {"records": out})
     hS, hL = S.copy(), L.copy()
     for _ in range(5):
         preint.preintegrate_host(1, hS, hL, synth.SIGMAS, 0, ns=wl["ns"])
@@ -620,7 +643,12 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the short runs of the other BASELINE configs appended to the default line")
     ap.add_argument("--distinct", type=int, default=0, help="generate only this many distinct windows on the host and tile them on the device (0 = all distinct)")
     ap.add_argument("--no-clocks", action="store_true", help="debug: do not poll nvidia-smi during the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     wl = WORKLOADS[args.workload]
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
@@ -629,16 +657,16 @@ def main():
     ctx = Ctx()
     if wl.get("factor"):
         if ctx.rank == 0:
-            run_factor(args, wl)
+            run_factor(args, wl, dump=args.dump_outputs)
         return
     if wl.get("single"):
         if ctx.rank == 0:
-            r = measure_single(ctx, args, wl)
-            r.update({"n_gpus": 1, "steps": 50, "warmup": 20, "ms_per_step": r["kernel_ms"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
-                      "dtype": "f64", "data": "synthetic", "gpu_launches": 50})
+            r = measure_single(ctx, args, wl, steps=args.steps, dump=args.dump_outputs)
+            r.update({"n_gpus": 1, "steps": args.steps, "warmup": 20, "ms_per_step": r["kernel_ms"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+                      "dtype": "f64", "data": "synthetic", "gpu_launches": args.steps})
             print(json.dumps(r), flush=True)
         return
-    out = measure_preint(ctx, args.workload, args, args.steps, args.warmup, distinct=args.distinct or None, e2e=True, cpu=True)
+    out = measure_preint(ctx, args.workload, args, args.steps, args.warmup, distinct=args.distinct or None, e2e=True, cpu=True, dump=args.dump_outputs)
 
     # ---- the other BASELINE configs, short runs, appended to the default line so that the driver's record carries them
     if args.workload == "v1_10k_200" and not args.no_configs:

@@ -58,8 +58,12 @@ def test_cuda_matches_oracle_seeded(cuda, oracle, model, flags):
 
 
 @pytest.mark.parametrize("model", [1, 2])
-def test_cuda_matches_reference_live(cuda, reference, model):
+def test_cuda_matches_reference_live(cuda, oracle, model):
+    """Against the compiled reference (oracle/_ref), or the C oracle where the reference was not built: the oracle is pinned to the
+    reference's golden records by test_oracle.py."""
     from cpi_b200 import preint
+    from oracle import oracle as om
+    reference = om.Reference() if om.Reference.available() else oracle
     S, L = synth.make_windows(500, 200 if model == 1 else 400, rate=200.0 if model == 1 else 400.0, first_window=123456)
     ns = S.shape[1]
     got = preint.preintegrate_host(model, S, L, synth.SIGMAS, 0, ns=ns)

@@ -55,7 +55,17 @@ def test_oracle_factor_matches_golden(oracle, golden, model):
     assert np.max(np.abs(oracle.retract(X, F[f"m{model}/xi"]) - F[f"m{model}/retracted"])) <= 1e-14
 
 
-def test_oracle_quat_ops_match_reference(oracle, reference):
+def test_oracle_quat_ops_match_reference(oracle, golden):
+    """Every golden record stores the reference's q = rot_2_quat(R) of its own R (CpiV1.h:358): the oracle's rot_2_quat must give the
+    same quaternion on all of them.  The other helpers are compared live when oracle/_ref/libcpi_ref.so is built."""
+    from oracle import oracle as om
+    G = golden["preint"]
+    for key in (k for k in G.files if "/records_" in k):
+        for rec in G[key]:
+            assert np.max(np.abs(oracle.rot_2_quat(rec[4:13]) - rec[0:4])) <= 1e-15, key
+    if not om.Reference.available():
+        return
+    reference = om.Reference()
     rng = np.random.default_rng(3)
     for _ in range(50):
         q = rng.normal(size=4); q /= np.linalg.norm(q)
