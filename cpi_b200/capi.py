@@ -28,6 +28,8 @@ SYMBOLS = {
     "cpi_imu_chain_assemble": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, ctypes.c_double, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "cpi_imu_chain_solve_workspace": (c_i64, [c_i64]),
     "cpi_imu_chain_solve": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "cpi_imu_chain_marginals_workspace": (c_i64, [c_i64]),
+    "cpi_imu_chain_marginals": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "cpi_predict_state_batch": (c_int, [c_int, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "cpi_retract_batch": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp]),
     "cpi_host_last_timing": (c_int, [c_vp, c_vp]),

@@ -455,6 +455,21 @@ int cpi_imu_chain_solve(int64_t n_states, const double* D, const double* E, cons
     return CPI_OK;
 }
 
+int64_t cpi_imu_chain_marginals_workspace(int64_t n_states) { return n_states < 0 ? (int64_t)CPI_EINVAL : cpi::chain_solve_workspace_bytes(n_states); }
+
+int cpi_imu_chain_marginals(int64_t n_states, const double* D, const double* E, double* S_diag, double* S_off, void* workspace, void* stream) {
+    if (n_states < 0) return fail(CPI_EINVAL, "negative count");
+    if (n_states == 0) return CPI_OK;
+    if (!D || !S_diag || (n_states > 1 && (!E || !workspace))) return fail(CPI_EINVAL, "null pointer argument");
+    DevInfo d;
+    int rc = device_info(d);
+    if (rc) return rc;
+    int launches = 0;
+    CU(cpi::chain_marginals_launch(n_states, D, E, S_diag, S_off, (double*)workspace, (cudaStream_t)stream, &launches));
+    g_launches += launches;
+    return CPI_OK;
+}
+
 int cpi_predict_state_batch(int model, int64_t n, const double* states_k, const double* records, const double* lin, double* states_k1, void* stream) {
     if (model != 1 && model != 2) return fail(CPI_EINVAL, "model must be 1 or 2 (got %d)", model);
     if (n < 0) return fail(CPI_EINVAL, "negative count");

@@ -46,6 +46,8 @@ cudaError_t chain_assemble_launch(int64_t nf, const double* G11, const double* G
                                   int diagonal_damping, const double* prior_info, const double* prior_rhs, double* D, double* E, double* rhs, cudaStream_t st);
 int64_t chain_solve_workspace_bytes(int64_t n_states);
 cudaError_t chain_solve_launch(int64_t n_states, const double* D, const double* E, const double* b, double* x, double* ws, cudaStream_t st, int* launches);
+cudaError_t chain_marginals_launch(int64_t n_states, const double* D, const double* E, double* S_diag, double* S_off, double* ws, cudaStream_t st,
+                                   int* launches);
 cudaError_t retract_launch(int64_t n, const double* states, const double* xi, double* out, cudaStream_t st);
 
 }  // namespace cpi

@@ -6,8 +6,13 @@
 //   block cyclic reduction: a Cholesky-based solve of that SPD block-tridiagonal system (15x15 blocks) in log2(n) parallel levels
 //                     instead of a 5 000-step sequential block recurrence: odd nodes are eliminated (one warp per node: Cholesky of the
 //                     diagonal block + 31 forward substitutions), even nodes receive the Schur complements (one warp per node).
+//   selected inversion: the same forward sweep without right-hand side, then from the root down, one warp per odd node, the diagonal and
+//                     first off-diagonal 15x15 blocks of A^-1 (marginal covariances of every keyframe and of adjacent pairs, what GTSAM's
+//                     Marginals::marginalCovariance / jointMarginalCovariance return) from the Cholesky factors and Lc^-1 E products the
+//                     sweep left in the workspace: no dense inverse, 3 ceil(log2 n) + 1 launches.
 // GTSAM is not part of the reference tree (bitbucket gtborg/gtsam @ c21186c): PARITY UNPINNED -- validated against dense / banded
-// CPU solves of the same system (tests/test_gpu_parity.py).
+// CPU solves of the same system (tests/test_gpu_parity.py) and, for the marginals, dense inverses and the forward-propagated covariance of
+// the chain (tests/test_chain_marginals.py).
 #include "cpi_common.cuh"
 #include "cpi_kernels.h"
 
@@ -50,6 +55,36 @@ CPI_DEV double warp_bwd15(const double* L, double r, int lane) {
         if (lane < k) r = fma(-L[k * 16 + lane], xk, r);          // (L^T)[lane, k] = L[k, lane]
     }
     return x;
+}
+
+// x = L^-T y  for a per-lane right-hand side held in registers (y -> x in place)
+CPI_DEV void bwd15(const double* L, double* y) {
+#pragma unroll
+    for (int i = 14; i >= 0; i--) {
+        double t = y[i];
+#pragma unroll
+        for (int k = i + 1; k < 15; k++) t = fma(-L[k * 16 + i], y[k], t);
+        y[i] = t / L[i * 16 + i];
+    }
+}
+// M = L^-1 into shared memory (column-major; lane c < 15 forms column c); ends with __syncwarp
+CPI_DEV void warp_inv_lower15(const double* L, double* M, int lane) {
+    if (lane < 15) {
+        double y[15];
+#pragma unroll
+        for (int i = 0; i < 15; i++) y[i] = (i == lane) ? 1.0 : 0.0;
+        fwd15(L, y);
+#pragma unroll
+        for (int i = 0; i < 15; i++) M[i + 15 * lane] = y[i];
+    }
+    __syncwarp();
+}
+// (L L^T)^-1 [a, b] = (M^T M)[a, b] with M = L^-1: entries (a, b) and (b, a) sum the same products in the same order, so the result is
+// exactly symmetric
+CPI_DEV double inv_entry15(const double* M, int a, int b) {
+    double s = 0.0;
+    for (int k = a > b ? a : b; k < 15; k++) s = fma(M[k + 15 * a], M[k + 15 * b], s);
+    return s;
 }
 
 // ---- explicitly whitened Jacobian form --------------------------------------------------------------------------------------------
@@ -128,6 +163,7 @@ __global__ void k_chain_assemble(int64_t nf, const double* G11, const double* G1
 // ---- block cyclic reduction ---------------------------------------------------------------------------------------------------------
 // Level with m nodes: row i reads  E[i-1]^T x_{i-1} + D[i] x_i + E[i] x_{i+1} = b[i].
 // Odd node i = 2t+1:  D_i = Lc Lc^T,  Za = Lc^-1 E[i-1]^T,  Zb = Lc^-1 E[i] (if i+1 < m),  zb = Lc^-1 b_i      (kept for the back-substitution)
+// b = NULL (the marginals need no right-hand side) skips zb.
 __global__ void __launch_bounds__(128) k_bcr_eliminate(int64_t m, const double* D, const double* E, const double* b, double* Lc, double* Za, double* Zb, double* zb) {
     __shared__ double sL[4][15 * 16];
     const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -140,7 +176,7 @@ __global__ void __launch_bounds__(128) k_bcr_eliminate(int64_t m, const double* 
     warp_chol15(L, lane);
     for (int k = lane; k < 225; k += 32) { const int r = k % 15, c = k / 15; Lc[t * 225 + k] = (r >= c) ? L[r * 16 + c] : 0.0; }
     const bool has_right = i + 1 < m;
-    if (lane < 31) {
+    if (lane < 30 || (lane == 30 && b)) {
         double y[15];
         if (lane < 15) {
 #pragma unroll
@@ -161,6 +197,7 @@ __global__ void __launch_bounds__(128) k_bcr_eliminate(int64_t m, const double* 
 
 // Even node j = 2u -> node u of the next level:
 //   D' = D_j - Zb_{j-1}^T Zb_{j-1} - Za_{j+1}^T Za_{j+1},   b' = b_j - Zb_{j-1}^T zb_{j-1} - Za_{j+1}^T zb_{j+1},   E' = -Za_{j+1}^T Zb_{j+1}  (couples x_j and x_{j+2})
+// b = NULL skips b'.
 __global__ void __launch_bounds__(128) k_bcr_reduce(int64_t m, const double* D, const double* b, const double* Za, const double* Zb, const double* zb,
                                                     double* Dn, double* En, double* bn) {
     __shared__ double sZ[4][4][225 + 15];      // [warp][ZbL | ZaR | ZbR | (zbL, zbR)]
@@ -176,7 +213,7 @@ __global__ void __launch_bounds__(128) k_bcr_reduce(int64_t m, const double* D, 
         ZaR[k] = hasR ? Za[tr * 225 + k] : 0.0;
         ZbR[k] = hasRR ? Zb[tr * 225 + k] : 0.0;
     }
-    if (lane < 15) { zz[lane] = hasL ? zb[tl * 15 + lane] : 0.0; zz[15 + lane] = hasR ? zb[tr * 15 + lane] : 0.0; }
+    if (lane < 15 && b) { zz[lane] = hasL ? zb[tl * 15 + lane] : 0.0; zz[15 + lane] = hasR ? zb[tr * 15 + lane] : 0.0; }
     __syncwarp();
     for (int k = lane; k < 225; k += 32) {
         const int r = k % 15, c = k / 15;                          // column-major 15x15; Z matrices are column-major: Z[q + 15 col]
@@ -190,7 +227,7 @@ __global__ void __launch_bounds__(128) k_bcr_reduce(int64_t m, const double* D, 
         Dn[u * 225 + k] = d;
         if (hasRR) En[u * 225 + k] = en;
     }
-    if (lane < 15) {
+    if (lane < 15 && b) {
         double v = b[j * 15 + lane];
 #pragma unroll
         for (int q = 0; q < 15; q++) { v = fma(-ZbL[q + 15 * lane], zz[q], v); v = fma(-ZaR[q + 15 * lane], zz[15 + q], v); }
@@ -243,6 +280,107 @@ __global__ void __launch_bounds__(128) k_bcr_backsub(int64_t m, int64_t stride, 
     if (lane < 15) x[i * stride * 15 + lane] = xv;
 }
 
+// ---- selected inversion: diagonal and first off-diagonal blocks of Sigma = A^-1 --------------------------------------------------------
+// Same forward sweep (without right-hand side), then level by level from the root down.  The coarse level's Sigma is the Sigma of the
+// finer level restricted to its even nodes (the inverse of a Schur complement is a block of the inverse).
+
+// last level (one node): Sigma = D^-1
+__global__ void k_bcr_root_inv(const double* D, double* S) {
+    __shared__ double L[15 * 16], M[225];
+    const int lane = threadIdx.x;
+    for (int k = lane; k < 225; k += 32) { const int r = k % 15, c = k / 15; if (r >= c) L[r * 16 + c] = D[k]; }
+    __syncwarp();
+    warp_chol15(L, lane);
+    warp_inv_lower15(L, M, lane);
+    for (int k = lane; k < 225; k += 32) S[k] = inv_entry15(M, k % 15, k / 15);
+}
+
+// Odd node i = 2t+1 of a level whose nodes sit at original indices i * stride.  Its neighbours l = i-1, r = i+1 are the coarse nodes t, t+1,
+// whose blocks Sigma_ll, Sigma_rr (in S) and Sigma_lr (the coarse off-diagonal block t, in Sc) the level above produced.  With
+// W_l = Lc^-T Za = D_i^-1 E[i-1]^T and W_r = Lc^-T Zb = D_i^-1 E[i] (zero without a right neighbour):
+//   Sigma_il = -(W_l Sigma_ll + W_r Sigma_lr^T),   Sigma_ir = -(W_l Sigma_lr + W_r Sigma_rr),   Sigma_ii = D_i^-1 - Sigma_il W_l^T - Sigma_ir W_r^T
+// Sigma_ii is written symmetrised.  Every adjacent pair of the level contains one odd node, so the pass writes the level's whole first
+// off-diagonal into So (block (k, k+1) at k, column-major; So = NULL: not wanted).
+__global__ void __launch_bounds__(128) k_bcr_selinv(int64_t m, int64_t stride, const double* Lc, const double* Za, const double* Zb, const double* Sc,
+                                                    double* S, double* So) {
+    __shared__ double sL[4][15 * 16], sT[4][5][225];   // [warp][W_l | W_r | Sigma_ll -> Sigma_il | Sigma_rr -> Sigma_ir | Sigma_lr -> Lc^-1 -> Sigma_ii]
+    const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t t = (int64_t)blockIdx.x * 4 + wib;
+    const int64_t i = 2 * t + 1;
+    if (i >= m) return;
+    const bool has_right = i + 1 < m;
+    double *L = sL[wib], *Wl = sT[wib][0], *Wr = sT[wib][1], *Xl = sT[wib][2], *Xr = sT[wib][3], *Y = sT[wib][4];
+    for (int k = lane; k < 225; k += 32) {
+        const int r = k % 15, c = k / 15;
+        if (r >= c) L[r * 16 + c] = Lc[t * 225 + k];
+        Xl[k] = S[(i - 1) * stride * 225 + k];
+        Xr[k] = has_right ? S[(i + 1) * stride * 225 + k] : 0.0;
+        Y[k] = has_right ? Sc[t * 225 + k] : 0.0;
+    }
+    __syncwarp();
+    if (lane < 30) {                                               // lanes 0..14: columns of W_l, 15..29: columns of W_r
+        const int c = lane < 15 ? lane : lane - 15;
+        double y[15];
+#pragma unroll
+        for (int r = 0; r < 15; r++) y[r] = lane < 15 ? Za[t * 225 + 15 * c + r] : (has_right ? Zb[t * 225 + 15 * c + r] : 0.0);
+        bwd15(L, y);
+        double* dst = (lane < 15 ? Wl : Wr) + 15 * c;
+#pragma unroll
+        for (int r = 0; r < 15; r++) dst[r] = y[r];
+    }
+    __syncwarp();
+    double vl[8], vr[8];                                           // entry k = lane + 32 s of Sigma_il / Sigma_ir (column-major)
+#pragma unroll
+    for (int s = 0; s < 8; s++) {
+        const int k = lane + 32 * s;
+        if (k < 225) {
+            const int a = k % 15, b = k / 15;
+            double xl = 0.0, xr = 0.0;
+#pragma unroll
+            for (int q = 0; q < 15; q++) {
+                xl = fma(-Wl[a + 15 * q], Xl[q + 15 * b], xl);
+                xl = fma(-Wr[a + 15 * q], Y[b + 15 * q], xl);
+                xr = fma(-Wl[a + 15 * q], Y[q + 15 * b], xr);
+                xr = fma(-Wr[a + 15 * q], Xr[q + 15 * b], xr);
+            }
+            vl[s] = xl; vr[s] = xr;
+        }
+    }
+    __syncwarp();
+#pragma unroll
+    for (int s = 0; s < 8; s++) {
+        const int k = lane + 32 * s;
+        if (k < 225) {
+            const int a = k % 15, b = k / 15;
+            Xl[k] = vl[s]; Xr[k] = vr[s];
+            if (So) {
+                So[(i - 1) * 225 + b + 15 * a] = vl[s];            // block (i-1, i) = Sigma_il^T
+                if (has_right) So[i * 225 + k] = vr[s];            // block (i, i+1) = Sigma_ir
+            }
+        }
+    }
+    warp_inv_lower15(L, Y, lane);                                  // (its __syncwarp also publishes Sigma_il / Sigma_ir)
+#pragma unroll
+    for (int s = 0; s < 8; s++) {
+        const int k = lane + 32 * s;
+        if (k < 225) {
+            const int a = k % 15, b = k / 15;
+            double d = inv_entry15(Y, a, b);
+#pragma unroll
+            for (int q = 0; q < 15; q++) {
+                d = fma(-Xl[a + 15 * q], Wl[b + 15 * q], d);
+                d = fma(-Xr[a + 15 * q], Wr[b + 15 * q], d);
+            }
+            vl[s] = d;
+        }
+    }
+    __syncwarp();
+#pragma unroll
+    for (int s = 0; s < 8; s++) { const int k = lane + 32 * s; if (k < 225) Y[k] = vl[s]; }
+    __syncwarp();
+    for (int k = lane; k < 225; k += 32) { const int a = k % 15, b = k / 15; S[i * stride * 225 + k] = 0.5 * (Y[k] + Y[b + 15 * a]); }
+}
+
 // ---- launchers ----------------------------------------------------------------------------------------------------------------------
 cudaError_t whiten_launch(int rd, int64_t n, const double* records, const double* e, const double* H1, const double* H2, double* A1, double* A2, double* b, cudaStream_t st) {
     if (n == 0) return cudaSuccess;
@@ -269,35 +407,59 @@ static int64_t bcr_doubles(int64_t m) {
 }
 int64_t chain_solve_workspace_bytes(int64_t n_states) { return bcr_doubles(n_states) * 8; }
 
-cudaError_t chain_solve_launch(int64_t n_states, const double* D, const double* E, const double* b, double* x, double* ws, cudaStream_t st, int* launches) {
-    struct Level { int64_t m; const double *D, *E, *b; double *Lc, *Za, *Zb, *zb; };
-    Level lv[64];
+struct BcrLevel { int64_t m; double *Lc, *Za, *Zb, *zb, *En; };   // En: the reduced E' this level produces (the next level's E)
+
+// forward sweep, two launches per level, down to one node; returns the number of levels and the root's D (and b)
+static int bcr_forward(int64_t n_states, const double* D, const double* E, const double* b, double* ws, cudaStream_t st, BcrLevel* lv,
+                       const double** root_D, const double** root_b) {
     int nl = 0;
     int64_t m = n_states;
     const double *cD = D, *cE = E, *cb = b;
     double* p = ws;
-    int nk = 0;
     while (m > 1) {
         const int64_t odd = m / 2, even = (m + 1) / 2;
-        Level& L = lv[nl++];
-        L.m = m; L.D = cD; L.E = cE; L.b = cb;
+        BcrLevel& L = lv[nl++];
+        L.m = m;
         L.Lc = p; p += odd * 225; L.Za = p; p += odd * 225; L.Zb = p; p += odd * 225; L.zb = p; p += odd * 15;
-        double* nD = p; p += even * 225; double* nE = p; p += even * 225; double* nb = p; p += even * 15;
+        double* nD = p; p += even * 225; L.En = p; p += even * 225; double* nb = p; p += even * 15;
         k_bcr_eliminate<<<(int)((odd + 3) / 4), 128, 0, st>>>(m, cD, cE, cb, L.Lc, L.Za, L.Zb, L.zb);
-        k_bcr_reduce<<<(int)((even + 3) / 4), 128, 0, st>>>(m, cD, cb, L.Za, L.Zb, L.zb, nD, nE, nb);
-        nk += 2;
-        cD = nD; cE = nE; cb = nb; m = even;
+        k_bcr_reduce<<<(int)((even + 3) / 4), 128, 0, st>>>(m, cD, cb, L.Za, L.Zb, L.zb, nD, L.En, nb);
+        cD = nD; cE = L.En; cb = b ? nb : nullptr; m = even;
     }
-    k_bcr_root<<<1, 32, 0, st>>>(cD, cb, x, 1);
-    nk++;
+    *root_D = cD; *root_b = cb;
+    return nl;
+}
+
+cudaError_t chain_solve_launch(int64_t n_states, const double* D, const double* E, const double* b, double* x, double* ws, cudaStream_t st, int* launches) {
+    BcrLevel lv[64];
+    const double *rD, *rb;
+    const int nl = bcr_forward(n_states, D, E, b, ws, st, lv, &rD, &rb);
+    k_bcr_root<<<1, 32, 0, st>>>(rD, rb, x, 1);
     int64_t stride = (int64_t)1 << nl;
     for (int l = nl - 1; l >= 0; l--) {
         stride >>= 1;
         const int64_t odd = lv[l].m / 2;
         k_bcr_backsub<<<(int)((odd + 3) / 4), 128, 0, st>>>(lv[l].m, stride, lv[l].Lc, lv[l].Za, lv[l].Zb, lv[l].zb, x);
-        nk++;
     }
-    if (launches) *launches = nk;
+    if (launches) *launches = 3 * nl + 1;
+    return cudaGetLastError();
+}
+
+// Same workspace as the solve.  A level's reduced E' is dead once the forward sweep is done; its slot then holds that level's Sigma
+// off-diagonal blocks (written by the level's selected-inversion pass, read by the next finer one).  Level 0's go to S_off.
+cudaError_t chain_marginals_launch(int64_t n_states, const double* D, const double* E, double* S_diag, double* S_off, double* ws, cudaStream_t st,
+                                   int* launches) {
+    BcrLevel lv[64];
+    const double *rD, *rb;
+    const int nl = bcr_forward(n_states, D, E, nullptr, ws, st, lv, &rD, &rb);
+    k_bcr_root_inv<<<1, 32, 0, st>>>(rD, S_diag);
+    int64_t stride = (int64_t)1 << nl;
+    for (int l = nl - 1; l >= 0; l--) {
+        stride >>= 1;
+        const int64_t odd = lv[l].m / 2;
+        k_bcr_selinv<<<(int)((odd + 3) / 4), 128, 0, st>>>(lv[l].m, stride, lv[l].Lc, lv[l].Za, lv[l].Zb, lv[l].En, S_diag, l > 0 ? lv[l - 1].En : S_off);
+    }
+    if (launches) *launches = 3 * nl + 1;
     return cudaGetLastError();
 }
 

@@ -4,7 +4,7 @@
     ImuFactorCPIv1 / ImuFactorCPIv2  gtsam/ImuFactorCPIv1.h:55, gtsam/ImuFactorCPIv2.h:55   (ctor argument order kept)
         .evaluateError(state_i, state_j, H1=False, H2=False)      gtsam/ImuFactorCPIv1.cpp:37, ImuFactorCPIv2.cpp:38
 
-and the batch entry points (``factor_eval``, ``predict_state``, ``retract``).  The residual and Jacobians are UNWHITENED,
+and the batch entry points (``factor_eval``, ``predict_state``, ``retract``, the chain solve and its marginal covariances).  The residual and Jacobians are UNWHITENED,
 exactly what evaluateError returns; GTSAM's Gaussian::Covariance(P_meas) whitening is outside the reference tree.
 All arithmetic happens in libcpi_b200.so on the GPU.
 """
@@ -154,7 +154,36 @@ def chain_solve(D, E, rhs, stream=None, workspace=None):
     return x
 
 
+def chain_marginals(D, E, want_off=True, workspace=None, stream=None):
+    """Marginal covariances of the chain (cpi_imu_chain_marginals): the diagonal blocks Sigma_kk and, with want_off, the blocks Sigma_k,k+1
+    of Sigma = A^-1 for A = tridiag(E^T, D, E), by selected inversion on the device.  Device tensors D [n+1,225], E [n,225].
+    Returns (S_diag [n+1,225], S_off [n,225] or None), column-major 15x15 blocks."""
+    import torch
+
+    lib = capi.load()
+    n = D.shape[0]
+    S_diag = torch.empty((n, 225), dtype=torch.float64, device=D.device)
+    S_off = torch.empty((max(n - 1, 0), 225), dtype=torch.float64, device=D.device) if want_off else None
+    nbytes = int(lib.cpi_imu_chain_marginals_workspace(n))
+    if workspace is None or workspace.numel() * 8 < nbytes:
+        workspace = torch.empty((nbytes + 7) // 8, dtype=torch.float64, device=D.device)
+    st = stream if stream is not None else torch.cuda.current_stream()
+    capi.check(lib.cpi_imu_chain_marginals(n, _tptr(D.contiguous()), _tptr(E.contiguous()), _tptr(S_diag), _tptr(S_off), _tptr(workspace),
+                                           ctypes.c_void_p(st.cuda_stream)))
+    return S_diag, S_off
+
+
 _PRIOR = {}
+
+
+def _prior_info(dev, prior_sigma):
+    """1/prior_sigma^2 I (15x15, flattened) on x_0, cached per device."""
+    import torch
+
+    key = (dev, prior_sigma)
+    if key not in _PRIOR:
+        _PRIOR[key] = (torch.eye(15, dtype=torch.float64, device=dev) / (prior_sigma * prior_sigma)).reshape(-1).contiguous()
+    return _PRIOR[key]
 
 
 def chain_lm_step(model, states, records, lin, lam=1e-5, prior_sigma=1e-4, stream=None, diagonal_damping=True):
@@ -163,17 +192,22 @@ def chain_lm_step(model, states, records, lin, lam=1e-5, prior_sigma=1e-4, strea
     reference initialises with cov = 1e-8 I, GraphSolver.cpp:331; Marquardt damping lam * diag by default, lam = GTSAM's lambdaInitial:
     an undamped IMU-only chain of thousands of keyframes is numerically singular in fp64) -> block-cyclic-reduction solve -> JPLNavState::retract.
     Returns (new_states, delta, cost = sum e^T P^-1 e before the step)."""
-    import torch
-
-    dev = states.device
-    key = (dev, prior_sigma)
-    if key not in _PRIOR:
-        _PRIOR[key] = (torch.eye(15, dtype=torch.float64, device=dev) / (prior_sigma * prior_sigma)).reshape(-1).contiguous()
     e, H1, H2 = factor_eval(model, states, records, lin, stream=stream)
     G11, G12, G22, g1, g2, f = factor_hessian(model, records, e, H1, H2, stream=stream)
-    D, E, rhs = chain_assemble(G11, G12, G22, g1, g2, lam, _PRIOR[key], None, stream=stream, diagonal_damping=diagonal_damping)
+    D, E, rhs = chain_assemble(G11, G12, G22, g1, g2, lam, _prior_info(states.device, prior_sigma), None, stream=stream, diagonal_damping=diagonal_damping)
     dx = chain_solve(D, E, rhs, stream=stream)
     return retract(states, dx, stream=stream), dx, f.sum()
+
+
+def chain_marginal_covariances(model, states, records, lin, prior_sigma=1e-4, stream=None):
+    """Marginal covariances of an IMU-only chain at ``states``, what GTSAM's Marginals computes at an estimate: the normal equations are
+    linearised there without damping (lambda = 0), with the x_0 prior of chain_lm_step, and inverted selectively on the device.
+    Returns (S_diag [n+1,225]: Sigma_kk, S_off [n,225]: Sigma_k,k+1), column-major 15x15 blocks in the error-state order.
+    An IMU-only chain anchored by one prior is numerically singular in fp64 beyond a few hundred keyframes (DESIGN.md section 5)."""
+    e, H1, H2 = factor_eval(model, states, records, lin, stream=stream)
+    G11, G12, G22, g1, g2, _ = factor_hessian(model, records, e, H1, H2, stream=stream)
+    D, E, _ = chain_assemble(G11, G12, G22, g1, g2, 0.0, _prior_info(states.device, prior_sigma), None, stream=stream)
+    return chain_marginals(D, E, stream=stream)
 
 
 def predict_state(model, states_k, records, lin, stream=None):

@@ -212,6 +212,25 @@ int64_t cpi_imu_chain_solve_workspace(int64_t n_states);
 int cpi_imu_chain_solve(int64_t n_states, const double* D, const double* E, const double* rhs,
                         double* x, void* workspace, void* stream);
 
+/*
+ * Marginal covariances of the chain: the diagonal and first off-diagonal 15x15 blocks of Sigma = A^-1 for the SPD block-tridiagonal
+ * A = tridiag(E^T, D, E) of cpi_imu_chain_assemble -- what GTSAM's Marginals::marginalCovariance(x_k) and the (x_k, x_k+1) block of
+ * jointMarginalCovariance return at the linearisation point (assemble with lambda = 0 for that).  Selected inversion by block cyclic
+ * reduction: the forward sweep of cpi_imu_chain_solve without right-hand side, then one pass per level from the root down, 3 ceil(log2 n) + 1
+ * kernel launches; no dense inverse is formed.
+ *   S_diag  device double[n_states * 225]      block k = Sigma_kk, column-major, exactly symmetric
+ *   S_off   device double[(n_states-1) * 225]  block k = Sigma_k,k+1 (column-major), or NULL when only the diagonal blocks are wanted
+ *   workspace  device buffer of cpi_imu_chain_marginals_workspace(n_states) bytes
+ * All pointers are DEVICE pointers; enqueued on `stream` without synchronising; n_states = 0 is a no-op.  A matrix that is not positive
+ * definite gives NaN outputs.  The NOTE above applies unchanged: an undamped IMU-only chain anchored by one prior is numerically singular in
+ * fp64 beyond a few hundred keyframes, and so are its covariances; the other factors of the real graph (or a prior per keyframe) make it
+ * well posed.  PARITY UNPINNED (GTSAM is not in the reference tree); validated against dense inverses, against the covariance the filter's
+ * forward propagation gives for a chain anchored at x_0 only, and against refined banded CPU solves.
+ */
+int64_t cpi_imu_chain_marginals_workspace(int64_t n_states);
+int cpi_imu_chain_marginals(int64_t n_states, const double* D, const double* E,
+                            double* S_diag, double* S_off, void* workspace, void* stream);
+
 /* ---- callers either side of the factor ("next" rows) ----------------------------------------------------------------- */
 
 /* x_{k+1} prediction from x_k and a record: getpredictedstate_v1/_v2 (GraphSolver_IMU.cpp:263-307).
